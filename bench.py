@@ -5,6 +5,7 @@
     python bench.py --config 3|4|5 ...                             # LoRA + IP-Adapter | ControlLora | SAM ViT-H
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference algorithm's CPU path (oracle port), host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one ``StableDiffusion_XL(x, step=..)`` call at latent batch 8 with classifier-free
 guidance (UNet batch 16): set contexts, sigma-scale, SDXLUNet forward, CFG combine, Euler update
@@ -54,6 +55,26 @@ T0 = time.time()
 
 def log(msg: str) -> None:
     print(f"[bench {time.time() - T0:7.1f}s] {msg}", file=sys.stderr, flush=True)
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir: str, outputs: dict[str, torch.Tensor]) -> None:
+    """Write each output as ``out_dir/<name>.npy`` in float32, so that two builds can be compared output for output.
+    Past DUMP_BYTES in all, each output is cut to the same fixed, seeded sample of its flattened elements."""
+    import numpy as np
+
+    path = Path(out_dir)
+    path.mkdir(parents=True, exist_ok=True)
+    total = 4 * sum(t.numel() for t in outputs.values())
+    for name, t in outputs.items():
+        values = t.detach().float().cpu()
+        if total > DUMP_BYTES:
+            keep = t.numel() * (DUMP_BYTES - 4096 * len(outputs)) // total
+            values = values.flatten()[torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values]
+        np.save(path / f"{name}.npy", values.numpy())
+    log(f"outputs of the last timed step written to {path}: {', '.join(outputs)}")
 
 
 def measured_peaks() -> tuple[dict, str]:
@@ -325,7 +346,7 @@ def run_config1(args) -> None:
     prev, oops.FAST = oops.FAST, True
     try:
         with no_grad():
-            repeats = max(5, min(args.steps, 10))
+            repeats = args.steps
             times = {}
             for name, fn in (("engine", engine), ("reference", reference)):
                 for _ in range(max(args.warmup, 1)):
@@ -337,6 +358,8 @@ def run_config1(args) -> None:
     finally:
         oops.FAST = prev
     (t_engine, y), (t_ref, y_ref) = times["engine"], times["reference"]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"unet_output": y})
     err = float((y - y_ref).abs().max() / y_ref.abs().max())
     if not err <= 1e-5:
         raise SystemExit(f"bench.py --config 1: host path differs from the reference's ATen evaluation by {err:.3e}")
@@ -618,10 +641,12 @@ def run_gpu_arm(args) -> None:
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
             for s in range(args.steps):
-                step_resident(s)
+                last = step_resident(s)
             e1.record()
             barrier()
         ms_total = max_over_ranks(e0.elapsed_time(e1))
+        if args.dump_outputs and rank == 0:  # before the e2e loop reuses the graph's output buffers
+            dump_outputs(args.dump_outputs, {"image_embeddings" if cfg == 5 else "latents": last})
         eager_launches = B.launch_count() - launches0
         graph_launches = (runner.replays - replays0) * runner.launches_per_replay if runner else 0
         gpu_launches = eager_launches + graph_launches
@@ -756,7 +781,14 @@ def main() -> None:
     ap.add_argument("--resident-only", action="store_true", help="stress mode: skip the e2e loop and the extras")
     ap.add_argument("--profile-step", action="store_true",
                     help="run ONE eager step between cudaProfilerStart/Stop and exit (for ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32; a fixed seeded "
+                         "sample when the outputs exceed 64 MB); inputs and weights are seeded, so runs with the same arguments compare")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.profile_step):
+        ap.error("--dump-outputs records the timed steps of the CUDA path (or of config 1)")
     if args.config == 1:
         run_config1(args)
         return

@@ -785,12 +785,197 @@ def main(write: bool) -> None:
             print(f"wrote {path.relative_to(ROOT)} ({path.stat().st_size / 1024:.0f} KiB, {len(tensors)} tensors)")
 
 
+TOKENIZER_TEXTS = [*PROMPTS, "naïve café — ünïcödé ☃ test_123 it's they're", "banana bandana " * 30, "<|startoftext|>hello<|endoftext|> world",
+                   "\t tabs\nand  newlines \x7f\x80"]
+LORA_SORT_KEYS = ["lora_unet_down_blocks_1_attentions_0_transformer_blocks_0_attn1_to_q", "lora_unet_down_blocks_10_attentions_0_proj_in",
+                  "a_to_out_0_lora", "plain_key", "lora_te_text_model_encoder_layers_3_self_attn_k_proj", "x_in", "y_out0"]
+SAM_FRAME_SIZES = ((1536, 768), (333, 517), (1024, 1024), (2000, 31))
+
+
+def pin_surface(write: bool) -> None:
+    """The reference's public surface, recorded for the structure and host-parity tests: repr() trees and state-dict
+    contracts of every model of the hot path before / after adapter injection, and digests of the outputs of the host-side
+    modules that must be bit-identical (structure.json.xz); and the CLIP merge table cut to the
+    48 894 ranks the tokenizer reads (clip_merges.txt.xz)."""
+    import gzip
+    import json
+    import lzma
+
+    rfl = _import_reference()
+    import numpy as np
+    from PIL import Image
+
+    import refiners
+    import refiners.foundationals.dinov2 as rdino
+    import refiners.foundationals.segment_anything.utils as rsam
+    from refiners.fluxion.adapters.lora import LinearLora as RLora, LoraAdapter as RAdapter
+    from refiners.fluxion.utils import gaussian_blur as rblur
+    from refiners.foundationals.clip.image_encoder import CLIPImageEncoder as REnc, CLIPImageEncoderH as REncH
+    from refiners.foundationals.clip.text_encoder import CLIPTextEncoderG, CLIPTextEncoderH, CLIPTextEncoderL
+    from refiners.foundationals.clip.tokenizer import CLIPTokenizer
+    from refiners.foundationals.latent_diffusion.auto_encoder import LatentDiffusionAutoencoder
+    from refiners.foundationals.latent_diffusion.cross_attention import CrossAttentionBlock2d
+    from refiners.foundationals.latent_diffusion.image_prompt import ImageProjection, IPAdapter, PerceiverResampler
+    from refiners.foundationals.latent_diffusion.lora import SDLoraManager
+    from refiners.foundationals.latent_diffusion.solvers import DDIM, Euler
+    from refiners.foundationals.latent_diffusion.stable_diffusion_1.controlnet import SD1ControlnetAdapter
+    from refiners.foundationals.latent_diffusion.stable_diffusion_1.self_attention_guidance import SD1SAGAdapter
+    from refiners.foundationals.latent_diffusion.stable_diffusion_1.unet import SD1UNet
+    from refiners.foundationals.latent_diffusion.stable_diffusion_xl.control_lora import ControlLoraAdapter
+    from refiners.foundationals.latent_diffusion.stable_diffusion_xl.image_prompt import SDXLIPAdapter
+    from refiners.foundationals.latent_diffusion.stable_diffusion_xl.self_attention_guidance import SDXLSAGAdapter
+    from refiners.foundationals.latent_diffusion.stable_diffusion_xl.text_encoder import DoubleTextEncoder
+    from refiners.foundationals.latent_diffusion.stable_diffusion_xl.unet import SDXLUNet
+    from refiners.foundationals.latent_diffusion.style_aligned import StyleAligned
+    from refiners.foundationals.segment_anything.image_encoder import SAMViTH
+
+    from oracle.weights import keyed_state_dict
+    from tests.test_lora_manager import Holder, checkpoint
+    from tests.test_reference_structure import contract, digest, tree
+
+    print("public surface: trees, contracts, host-side outputs")
+    trees: dict[str, dict] = {}
+    values: dict = {}
+
+    def snap(name: str, module) -> None:
+        trees[name] = {"tree": tree(module), "contract": [[k, list(s)] for k, s in contract(module)]}
+
+    # SD 1.5 UNet + ControlNet, SDXL UNet + ControlLora + IP-Adapter
+    unet = SD1UNet(4, device="meta")
+    snap("sd1.unet", unet)
+    adapter = SD1ControlnetAdapter(unet, name="canny", scale=0.9).inject()
+    snap("sd1.unet.controlnet", unet), snap("sd1.controlnet", adapter)
+    adapter.eject()
+    snap("sd1.unet.controlnet_ejected", unet)
+    unet = SDXLUNet(4, device="meta")
+    snap("sdxl.unet", unet)
+    adapter = ControlLoraAdapter("canny", unet, scale=0.8).inject()
+    snap("sdxl.unet.control_lora", unet)
+    adapter.eject()
+    snap("sdxl.unet.control_lora_ejected", unet)
+    ip = SDXLIPAdapter(unet, scale=0.5)
+    ip.inject()
+    snap("sdxl.unet.ip_adapter", unet), snap("sdxl.ip_adapter.image_proj", ip.image_proj)
+    ip.eject()
+    snap("sdxl.unet.ip_adapter_ejected", unet)
+
+    def keyed(module, seed: int):
+        module.load_state_dict(keyed_state_dict({k: tuple(v.shape) for k, v in module.state_dict().items()}, seed=seed))
+        return module
+
+    # IP-Adapter plus: the PerceiverResampler's structure and numbers (keyed weights, seeded input)
+    snap("perceiver.image_proj", SDXLIPAdapter(SDXLUNet(4, device="meta"), fine_grained=True).image_proj)
+    resampler = keyed(PerceiverResampler(latents_dim=64, num_attention_layers=2, num_attention_heads=4, head_dim=16, num_tokens=5, input_dim=48,
+                                         output_dim=40), 31)
+    with torch.no_grad():
+        values["perceiver.y"] = digest(resampler(torch.randn(3, 11, 48, generator=torch.Generator().manual_seed(0))))
+
+    # CLIP image encoder H and the IP-Adapter's image -> context path on a tiny tower
+    enc_h = REncH(device="meta")
+    snap("clip.image_encoder_h", enc_h), snap("clip.image_encoder_h.grid", IPAdapter.convert_to_grid_features(enc_h))
+    enc = keyed(REnc(image_size=32, embedding_dim=48, output_dim=24, patch_size=8, num_layers=2, num_attention_heads=3, feedforward_dim=96), 32)
+    proj = keyed(ImageProjection(clip_image_embedding_dim=24, clip_text_embedding_dim=40), 33)
+    target = rfl.Chain(CrossAttentionBlock2d(channels=64, context_embedding_dim=40, context_key="ctx", num_attention_heads=2, use_linear_projection=True))
+    ip = IPAdapter(target, enc, proj)
+    images = torch.randn(3, 3, 32, 32, generator=torch.Generator().manual_seed(0))
+    with torch.no_grad():
+        values["clip.encoded"] = digest(enc(images))
+        for i, kwargs in enumerate(({}, {"weights": [1.0, 0.5, 2.0]}, {"concat_batches": False})):
+            values[f"clip.embedding.{i}"] = digest(ip.compute_clip_image_embedding(images, **kwargs))
+
+    # two LoRAs on every Linear of a cross-attention block
+    block = rfl.Chain(CrossAttentionBlock2d(channels=64, context_embedding_dim=48, context_key="ctx", num_attention_heads=2, num_attention_layers=2,
+                                            use_linear_projection=True, device="meta"))
+    snap("lora.block", block)
+    for lin, parent in list(block.walk(rfl.Linear, recurse=True)):
+        loras = [RLora(f"l{j}", in_features=lin.in_features, out_features=lin.out_features, rank=4, scale=s, device="meta") for j, s in enumerate((1.0, 1.4))]
+        RAdapter(lin, *loras).inject(parent)
+    snap("lora.block.loras", block)
+
+    snap("sam.vit_h", SAMViTH(device="meta"))
+    snap("vae", LatentDiffusionAutoencoder(device="meta"))
+    for name in ("DINOv2_small", "DINOv2_base_reg", "DINOv2_large", "DINOv2_giant_reg"):
+        snap(f"dinov2.{name}", getattr(rdino, name)(device="meta"))
+    for tag, solver in (("euler", Euler(num_inference_steps=30)), ("ddim", DDIM(num_inference_steps=20))):
+        for table in ("timesteps", "cumulative_scale_factors", "noise_std"):
+            values[f"solver.{tag}.{table}"] = digest(getattr(solver, table))
+
+    # self-attention guidance on SD 1.5 and SDXL, and the blur it uses
+    for tag, unet_cls, sag_cls in (("sd1", SD1UNet, SD1SAGAdapter), ("sdxl", SDXLUNet, SDXLSAGAdapter)):
+        unet = unet_cls(4, device="meta")
+        sag = sag_cls(unet, scale=0.3, kernel_size=7, sigma=1.5).inject()
+        snap(f"sag.{tag}.unet", unet), snap(f"sag.{tag}.adapter", sag)
+        values[f"sag.{tag}.settings"] = [sag.scale, sag.kernel_size, sag.sigma]
+        values[f"sag.{tag}.context_keys"] = sorted(sag.init_context().keys())
+        sag.eject()
+        snap(f"sag.{tag}.unet.ejected", unet)
+    x = torch.randn(1, 4, 16, 20, generator=torch.Generator().manual_seed(0))
+    for i, (size, sigma) in enumerate(((9, 1.0), ((3, 7), None), (5, (0.8, 2.0)))):
+        values[f"sag.blur.{i}"] = digest(rblur(x, size, sigma))
+
+    # CLIP tokenizer and text towers
+    tokenizer = CLIPTokenizer()
+    values["tokenizer.texts"] = TOKENIZER_TEXTS
+    for i, text in enumerate(TOKENIZER_TEXTS):
+        values[f"tokenizer.text.{i}"] = digest(tokenizer(text))
+    values["tokenizer.batch"], values["tokenizer.encode"] = digest(tokenizer(TOKENIZER_TEXTS[:4])), digest(tokenizer.encode("hello world"))
+    mapping = json.dumps(tokenizer.token_to_id_mapping, sort_keys=True, ensure_ascii=False).encode()
+    values["tokenizer.mapping_sha256"] = __import__("hashlib").sha256(mapping).hexdigest()
+    for cls in (CLIPTextEncoderL, CLIPTextEncoderH, CLIPTextEncoderG, DoubleTextEncoder):
+        snap(f"text.{cls.__name__}", cls(device="meta"))
+
+    # SDLoraManager on SD 1.5
+    values["lora_manager.sort_keys"] = {key: list(SDLoraManager.sort_keys(key)) for key in LORA_SORT_KEYS}
+    unet = SD1UNet(4, device="meta")
+    manager = SDLoraManager(Holder(unet, rfl.Chain()))
+    tensors = checkpoint(unet, rfl)
+    values["lora_manager.checkpoint_keys"] = list(tensors)
+
+    def lines(u) -> list[str]:  # the Lambda line prints a function signature whose annotations differ (jaxtyping): not structure
+        return [line for line in repr(u).splitlines() if "Lambda(compute_sinusoidal_embedding" not in line]
+
+    for name, scale in (("a", 0.4), ("b", 1.0)):
+        manager.add_loras(name, tensors=tensors, scale=scale)
+    values["lora_manager.names"], values["lora_manager.scales"] = sorted(manager.names), manager.scales
+    values["lora_manager.weights_a"], values["lora_manager.tree.added"] = list(manager.get_lora_weights("a")), lines(unet)
+    manager.remove_loras("a")
+    values["lora_manager.tree.removed_a"] = lines(unet)
+    manager.remove_all()
+    values["lora_manager.tree.removed_all"] = lines(unet)
+
+    # StyleAligned's shared-attention chain in every dtype
+    for dtype in (torch.float32, torch.bfloat16, torch.float16):
+        x = (torch.randn(6, 10, 16, generator=torch.Generator().manual_seed(0)) * 2 + 0.3).to(dtype)
+        for i, (adain, concatenate) in enumerate(((True, False), (True, True), (False, True), (False, False))):
+            values[f"style.{dtype}.{i}"] = digest(StyleAligned(adain, concatenate, 0.7)(x))
+
+    # SAM pre- / post-processing on odd sizes
+    rng, gen = np.random.default_rng(0), torch.Generator().manual_seed(0)
+    for w, h in SAM_FRAME_SIZES:
+        image = Image.fromarray(rng.integers(0, 255, (h, w, 3), dtype=np.uint8))
+        values[f"sam.{w}x{h}.scaled_size"] = list(rsam.compute_scaled_size((h, w), 1024))
+        masks, points = torch.randn(2, 3, 256, 256, generator=gen), torch.rand(2, 5, 2, generator=gen) * torch.tensor([w, h])
+        values[f"sam.{w}x{h}.preprocess"] = digest(rsam.preprocess_image(image, 1024))
+        values[f"sam.{w}x{h}.postprocess"] = digest(rsam.postprocess_masks(masks, (h, w), 1024))
+        values[f"sam.{w}x{h}.coordinates"] = digest(rsam.normalize_coordinates(points.clone(), (h, w), 1024))
+
+    if write:
+        with lzma.open(GOLDEN / "structure.json.xz", "wt", preset=9) as f:
+            json.dump({"trees": trees, "values": values}, f, ensure_ascii=False)
+        with gzip.open(Path(refiners.__file__).parent / "foundationals/clip/bpe_simple_vocab_16e6.txt.gz", "rt") as f:
+            merges = f.read().split("\n")[: 49152 - 256 - 2 + 1]
+        with lzma.open(GOLDEN / "clip_merges.txt.xz", "wt", encoding="utf-8", preset=9 | lzma.PRESET_EXTREME) as f:
+            f.write("\n".join(merges))
+        for name in ("structure.json.xz", "clip_merges.txt.xz"):
+            print(f"  wrote tests/golden/{name} ({(GOLDEN / name).stat().st_size / 1024:.0f} KiB)")
+
+
 if __name__ == "__main__":
     write = "--check" not in sys.argv
     sections = {
         "--only-controlnet": pin_controlnet, "--only-step": pin_denoise_step, "--only-vae": pin_vae, "--only-vae-tiled": pin_vae_tiled, "--only-dinov2": pin_dinov2,
         "--only-clip": pin_clip, "--only-clip-text": pin_clip_text, "--only-sag": pin_sag, "--only-t2i": pin_t2i, "--only-style-aligned": pin_style_aligned,
-        "--only-full-size": pin_full_size,
+        "--only-full-size": pin_full_size, "--only-surface": pin_surface,
     }
     chosen = [fn for flag, fn in sections.items() if flag in sys.argv]
     if chosen:

@@ -4,6 +4,10 @@ host path (fp32, <= 1e-5 relative) and the same graphs on the CUDA kernels - fp3
 criterion of tests/test_full_size_gpu.py (error vs the reference's fp32 output no larger than that of torch-eager bf16 on
 the same GPU + 1e-3 max|ref|)."""
 
+import gzip
+import hashlib
+import json
+import lzma
 from pathlib import Path
 
 import pytest
@@ -112,7 +116,6 @@ def test_vision_tower_gpu(cuda_device, case, dtype):
 
 
 # ------------------------------------------------------------------------------------------ CLIP text towers
-REF = Path("/root/reference/src/refiners")
 PROMPTS = ["a photo of a cat", "", "An astronaut riding a horse on Mars, 4k, highly-detailed!!"]
 
 
@@ -138,37 +141,38 @@ def test_clip_text_encoder_host():
     assert e_max <= 1e-5 and o_max <= 1e-5, (e_max, o_max)
 
 
-@pytest.mark.skipif(not REF.exists(), reason="/root/reference is not mounted here (the BPE merge table ships with it)")
-def test_clip_tokenizer_against_the_reference():
-    from oracle.pin_against_reference import _import_reference
+@pytest.fixture(scope="module")
+def vocabulary(tmp_path_factory) -> Path:
+    """The CLIP merge table (data published with OpenAI CLIP), cut to the ranks the tokenizer reads and stored as xz; the
+    tokenizer reads it gzipped, as it is published."""
+    path = tmp_path_factory.mktemp("clip") / "bpe_simple_vocab_16e6.txt.gz"
+    with lzma.open(GOLDEN / "clip_merges.txt.xz", "rb") as src, gzip.open(path, "wb") as dst:
+        dst.write(src.read())
+    return path
 
-    _import_reference()
-    from refiners.foundationals.clip.tokenizer import CLIPTokenizer as Theirs
 
+def test_clip_tokenizer_against_the_reference(vocabulary):
+    """Token ids, the token -> id table and the text towers' structure against the reference's recording."""
     from refiners_b200.foundationals.clip import CLIPTokenizer
-    from tests.test_reference_structure import same
+    from tests.test_reference_structure import digest, recorded_values, same
 
-    vocabulary = REF / "foundationals/clip/bpe_simple_vocab_16e6.txt.gz"
-    mine, theirs = CLIPTokenizer(vocabulary_path=vocabulary), Theirs()
+    mine = CLIPTokenizer(vocabulary_path=vocabulary)
     f = load_file(str(GOLDEN / "clip_text.safetensors"))
     assert torch.equal(mine(PROMPTS), f["l.tokens"]) and torch.equal(CLIPTokenizer(vocabulary_path=vocabulary, pad_token_id=0)(PROMPTS), f["xl.tokens_g"])
-    texts = [*PROMPTS, "naïve café — ünïcödé ☃ test_123 it's they're", "banana bandana " * 30, "<|startoftext|>hello<|endoftext|> world",
-             "\t tabs\nand  newlines \x7f\x80"]
-    for text in texts:
-        assert torch.equal(mine(text), theirs(text)), text
-    assert torch.equal(mine(texts[:4]), theirs(texts[:4])) and torch.equal(mine.encode("hello world"), theirs.encode("hello world"))
-    assert mine.token_to_id_mapping == theirs.token_to_id_mapping
+    texts = recorded_values("tokenizer.texts")
+    for i, text in enumerate(texts):
+        assert digest(mine(text)) == recorded_values(f"tokenizer.text.{i}"), text
+    assert digest(mine(texts[:4])) == recorded_values("tokenizer.batch") and digest(mine.encode("hello world")) == recorded_values("tokenizer.encode")
+    mapping = json.dumps(mine.token_to_id_mapping, sort_keys=True, ensure_ascii=False).encode()
+    assert hashlib.sha256(mapping).hexdigest() == recorded_values("tokenizer.mapping_sha256")
     # trees and state-dict contract of the towers and of SDXL's double encoder (pooling adapter injected)
-    from refiners.foundationals.clip.text_encoder import CLIPTextEncoderG as RG, CLIPTextEncoderH as RH, CLIPTextEncoderL as RL
-    from refiners.foundationals.latent_diffusion.stable_diffusion_xl.text_encoder import DoubleTextEncoder as RD
-
     from refiners_b200.foundationals.clip import CLIPTextEncoderG, CLIPTextEncoderH, CLIPTextEncoderL
     from refiners_b200.foundationals.latent_diffusion.stable_diffusion_xl.text_encoder import DoubleTextEncoder
 
-    for ours, ref in ((CLIPTextEncoderL, RL), (CLIPTextEncoderH, RH), (CLIPTextEncoderG, RG), (DoubleTextEncoder, RD)):
-        same(ours(device="meta"), ref(device="meta"))
+    for ours in (CLIPTextEncoderL, CLIPTextEncoderH, CLIPTextEncoderG, DoubleTextEncoder):
+        same(ours(device="meta"), f"text.{ours.__name__}")
     twin = DoubleTextEncoder(device="meta").structural_copy()
-    same(twin, RD(device="meta"))
+    same(twin, "text.DoubleTextEncoder")
 
 
 def test_prompt_embedding_api():

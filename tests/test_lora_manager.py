@@ -1,11 +1,8 @@
 """SDLoraManager (SURVEY.md section 2 #10): named LoRA sets on a Stable Diffusion UNet.
 
-Stand-alone behaviour (names, scales, removal, the "already exists" / "subset" assertions) and - where
-/root/reference is mounted - the same operations on the real reference must yield the same module tree, the same
-exported weight keys and the same checkpoint-key ordering."""
-
-import sys
-from pathlib import Path
+Stand-alone behaviour (names, scales, removal, the "already exists" / "subset" assertions) and the same operations as
+recorded on the reference (tests/golden/structure.json.xz): the same module tree, the same exported weight keys and the
+same checkpoint-key ordering."""
 
 import pytest
 import torch
@@ -61,32 +58,25 @@ def test_manager_add_scale_remove():
     assert manager.names == [] and repr(unet) == pristine
 
 
-@pytest.mark.skipif(not Path("/root/reference/src").exists(), reason="/root/reference is not mounted here")
 def test_manager_matches_the_reference():
-    from oracle.pin_against_reference import _import_reference
+    from tests.test_reference_structure import recorded_values
 
-    rfl = _import_reference()
-    from refiners.foundationals.latent_diffusion.lora import SDLoraManager as RefManager
-    from refiners.foundationals.latent_diffusion.stable_diffusion_1.unet import SD1UNet as RefUNet
-
-    for key in ("lora_unet_down_blocks_1_attentions_0_transformer_blocks_0_attn1_to_q", "lora_unet_down_blocks_10_attentions_0_proj_in",
-                "a_to_out_0_lora", "plain_key", "lora_te_text_model_encoder_layers_3_self_attn_k_proj", "x_in", "y_out0"):
-        assert SDLoraManager.sort_keys(key) == RefManager.sort_keys(key), key
-    ours, theirs = SD1UNet(4, device="meta"), RefUNet(4, device="meta")
-    mine, ref = SDLoraManager(Holder(ours)), RefManager(Holder(theirs, rfl.Chain()))
-    tensors = checkpoint(theirs, rfl)
-    assert list(tensors) == list(checkpoint(ours, fl))
+    for key, want in recorded_values("lora_manager.sort_keys").items():
+        assert list(SDLoraManager.sort_keys(key)) == want, key
+    ours = SD1UNet(4, device="meta")
+    mine = SDLoraManager(Holder(ours))
+    tensors = checkpoint(ours, fl)
+    assert list(tensors) == recorded_values("lora_manager.checkpoint_keys")
 
     def tree(unet):  # the Lambda line prints a function signature whose annotations differ (jaxtyping): not structure
         return [line for line in repr(unet).splitlines() if "Lambda(compute_sinusoidal_embedding" not in line]
 
     for name, scale in (("a", 0.4), ("b", 1.0)):
         mine.add_loras(name, tensors=tensors, scale=scale)
-        ref.add_loras(name, tensors=tensors, scale=scale)
-    assert sorted(mine.names) == sorted(ref.names) and mine.scales == ref.scales
-    assert list(mine.get_lora_weights("a")) == list(ref.get_lora_weights("a"))
-    assert tree(ours) == tree(theirs)
-    mine.remove_loras("a"); ref.remove_loras("a")
-    assert tree(ours) == tree(theirs)
-    mine.remove_all(); ref.remove_all()
-    assert tree(ours) == tree(theirs)
+    assert sorted(mine.names) == recorded_values("lora_manager.names") and mine.scales == recorded_values("lora_manager.scales")
+    assert list(mine.get_lora_weights("a")) == recorded_values("lora_manager.weights_a")
+    assert tree(ours) == recorded_values("lora_manager.tree.added")
+    mine.remove_loras("a")
+    assert tree(ours) == recorded_values("lora_manager.tree.removed_a")
+    mine.remove_all()
+    assert tree(ours) == recorded_values("lora_manager.tree.removed_all")

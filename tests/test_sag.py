@@ -19,7 +19,6 @@ from refiners_b200.foundationals.latent_diffusion import SD1UNet, SDXLUNet, Stab
 from refiners_b200.foundationals.latent_diffusion.solvers import DDIM
 
 GOLDEN = Path(__file__).parent / "golden"
-REF = Path("/root/reference/src/refiners")
 CASES = ((3, 7.5), (20, 5.0))
 
 
@@ -70,33 +69,26 @@ def test_gaussian_blur_is_a_normalised_reflecting_filter():
     assert torch.allclose(gaussian_blur(x, 9, 1.0), osag.gaussian_blur(x, 9, 1.0), atol=1e-6)
 
 
-@pytest.mark.skipif(not REF.exists(), reason="/root/reference is not mounted here")
 def test_structure_against_the_reference():
-    """Trees with the probes in place, the adapter's own tree, and what eject leaves behind - SD 1.5 and SDXL."""
-    from oracle.pin_against_reference import _import_reference
-    from tests.test_reference_structure import same, tree
-
-    _import_reference()
-    from refiners.foundationals.latent_diffusion.stable_diffusion_1.self_attention_guidance import SD1SAGAdapter as R1
-    from refiners.foundationals.latent_diffusion.stable_diffusion_1.unet import SD1UNet as RUNet1
-    from refiners.foundationals.latent_diffusion.stable_diffusion_xl.self_attention_guidance import SDXLSAGAdapter as RXL
-    from refiners.foundationals.latent_diffusion.stable_diffusion_xl.unet import SDXLUNet as RUNetXL
-    from refiners.fluxion.utils import gaussian_blur as rblur
+    """Trees with the probes in place, the adapter's own tree, and what eject leaves behind - SD 1.5 and SDXL - against the
+    reference's recording (tests/golden/structure.json.xz)."""
+    from tests.test_reference_structure import digest, recorded_values, same, same_tree
 
     from refiners_b200.foundationals.latent_diffusion.stable_diffusion_1.self_attention_guidance import SD1SAGAdapter
     from refiners_b200.foundationals.latent_diffusion.stable_diffusion_xl.self_attention_guidance import SDXLSAGAdapter
 
-    for mine_cls, ref_cls, mine_ad, ref_ad in ((SD1UNet, RUNet1, SD1SAGAdapter, R1), (SDXLUNet, RUNetXL, SDXLSAGAdapter, RXL)):
-        mine, theirs = mine_cls(4, device="meta"), ref_cls(4, device="meta")
-        a, b = mine_ad(mine, scale=0.3, kernel_size=7, sigma=1.5).inject(), ref_ad(theirs, scale=0.3, kernel_size=7, sigma=1.5).inject()
-        same(mine, theirs)
-        assert tree(a) == tree(b) and (a.scale, a.kernel_size, a.sigma) == (b.scale, b.kernel_size, b.sigma)
-        assert a.init_context().keys() == b.init_context().keys()
-        a.eject(), b.eject()
-        same(mine, theirs)
-    x = torch.randn(1, 4, 16, 20)
-    for size, sigma in ((9, 1.0), ((3, 7), None), (5, (0.8, 2.0))):
-        assert torch.equal(gaussian_blur(x, size, sigma), rblur(x, size, sigma))
+    for tag, mine_cls, mine_ad in (("sd1", SD1UNet, SD1SAGAdapter), ("sdxl", SDXLUNet, SDXLSAGAdapter)):
+        mine = mine_cls(4, device="meta")
+        a = mine_ad(mine, scale=0.3, kernel_size=7, sigma=1.5).inject()
+        same(mine, f"sag.{tag}.unet")
+        same_tree(a, f"sag.{tag}.adapter")
+        assert [a.scale, a.kernel_size, a.sigma] == recorded_values(f"sag.{tag}.settings")
+        assert sorted(a.init_context().keys()) == recorded_values(f"sag.{tag}.context_keys")
+        a.eject()
+        same(mine, f"sag.{tag}.unet.ejected")
+    x = torch.randn(1, 4, 16, 20, generator=torch.Generator().manual_seed(0))
+    for i, (size, sigma) in enumerate(((9, 1.0), ((3, 7), None), (5, (0.8, 2.0)))):
+        assert digest(gaussian_blur(x, size, sigma)) == recorded_values(f"sag.blur.{i}")
 
 
 # ------------------------------------------------------------------------------------------------ GPU

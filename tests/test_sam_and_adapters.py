@@ -283,25 +283,20 @@ def test_conv2d_lora_gpu(cuda_device, dtype, stride):
     check(y, ref, dtype)
 
 
-@pytest.mark.skipif(not __import__("pathlib").Path("/root/reference/src/refiners").exists(), reason="/root/reference is not mounted here")
 def test_sam_image_frame_matches_the_reference():
-    """Pre- / post-processing around the encoder (segment_anything/utils.py:7-130): bit-identical to the reference on odd sizes."""
+    """Pre- / post-processing around the encoder (segment_anything/utils.py:7-130): bit-identical to the reference's
+    recording on odd sizes."""
     import numpy as np
     from PIL import Image
 
-    from oracle.pin_against_reference import _import_reference
-
-    _import_reference()
-    import refiners.foundationals.segment_anything.utils as theirs
-
     import refiners_b200.foundationals.segment_anything.utils as mine
+    from tests.test_reference_structure import digest, recorded_values
 
-    rng = np.random.default_rng(0)
+    rng, gen = np.random.default_rng(0), torch.Generator().manual_seed(0)
     for w, h in ((1536, 768), (333, 517), (1024, 1024), (2000, 31)):
         image = Image.fromarray(rng.integers(0, 255, (h, w, 3), dtype=np.uint8))
-        assert mine.compute_scaled_size((h, w), 1024) == theirs.compute_scaled_size((h, w), 1024)
-        assert torch.equal(mine.preprocess_image(image, 1024), theirs.preprocess_image(image, 1024))
-        masks = torch.randn(2, 3, 256, 256)
-        assert torch.equal(mine.postprocess_masks(masks, (h, w), 1024), theirs.postprocess_masks(masks, (h, w), 1024))
-        points = torch.rand(2, 5, 2) * torch.tensor([w, h])
-        assert torch.equal(mine.normalize_coordinates(points.clone(), (h, w), 1024), theirs.normalize_coordinates(points.clone(), (h, w), 1024))
+        assert list(mine.compute_scaled_size((h, w), 1024)) == recorded_values(f"sam.{w}x{h}.scaled_size")
+        masks, points = torch.randn(2, 3, 256, 256, generator=gen), torch.rand(2, 5, 2, generator=gen) * torch.tensor([w, h])
+        assert digest(mine.preprocess_image(image, 1024)) == recorded_values(f"sam.{w}x{h}.preprocess"), (w, h)
+        assert digest(mine.postprocess_masks(masks, (h, w), 1024)) == recorded_values(f"sam.{w}x{h}.postprocess"), (w, h)
+        assert digest(mine.normalize_coordinates(points.clone(), (h, w), 1024)) == recorded_values(f"sam.{w}x{h}.coordinates"), (w, h)
